@@ -21,6 +21,10 @@ CG reduced-KKT solver, scaling=0, fixed rho, EmptyAccelerator (BASELINE.md 2).
 
 `--impl reference` times the oracle port for the same K steps / W warm-up (the reference itself cannot run
 here: no Julia; it has no C sources to compile).
+
+`--dump-outputs DIR` writes the x, s, mu and objective of the timed solve (after exactly --steps iterations from a cold
+start) as float64 .npy files, 2 MB at the default size: the problem comes from --seed, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -51,7 +55,14 @@ def parse_args():
     ap.add_argument("--seed", type=int, default=2)
     ap.add_argument("--cpu-sample-iters", type=int, default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed solve returned (x, s, mu, obj_val) as float64 DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the engine's outputs (--impl b200)")
+    return a
 
 
 def workload_config(a, extra=None):
@@ -268,6 +279,10 @@ def main():
     out = run(a.steps)
     barrier()
     dev_s = out.times["iter_time_device"]
+    if out.iter != a.steps:
+        raise SystemExit("the timed solve stopped after %d of %d iterations (%s)" % (out.iter, a.steps, out.status))
+    # the arrays the timed solve handed back; the later legs reuse the same host buffers
+    result = {"x": ox.copy(), "s": os_.copy(), "mu": omu.copy(), "obj_val": np.array(out.obj_val)}
     # ---- timed: end to end through the C ABI with host buffers ----------------------------------
     st = cosmo_b200.Settings(scaling=0, adaptive_rho=False, max_iter=a.steps, eps_abs=0.0, eps_rel=0.0).to_struct()
     eng.update_settings(st)
@@ -377,8 +392,27 @@ def main():
                                       "(P, q, A, b, K) at full size" % k_par,
                               "value": rel, "bound": 1e-8, "ok": bool(rel is not None and rel <= 1e-8)}
         print(json.dumps(line))
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, result, shard, m, dist)
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(path, result, shard, m, dist):
+    """Rank 0 writes `result` as float64 .npy files; each rank's s and mu hold only its own rows, so under sharding
+    they are gathered into the full m-vectors first (x and obj_val are the same on every rank)."""
+    if dist is not None:
+        parts = [None] * dist.get_world_size()
+        dist.all_gather_object(parts, (shard.rows, result["s"], result["mu"]))
+        for k, name in ((1, "s"), (2, "mu")):
+            full = np.empty(m)
+            for p in parts:
+                full[p[0]] = p[k]
+            result[name] = full
+    if shard.rank == 0:
+        os.makedirs(path, exist_ok=True)
+        for name, v in result.items():
+            np.save(os.path.join(path, name + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 if __name__ == "__main__":
