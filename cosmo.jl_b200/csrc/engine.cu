@@ -31,6 +31,7 @@
 #include "vector_kernels.cuh"
 #include "ruiz.cuh"
 #include "cg_persistent.cuh"
+#include "direct.cuh"
 
 namespace cosmo {
 
@@ -202,6 +203,7 @@ class EngineBase {
   virtual void get_rho_vec(void* out) = 0;
   virtual void get_w(void* out) = 0;
   virtual void psd_stats(int64_t* out8) = 0;
+  virtual void kkt_factor_stats(int64_t* factorizations, double* seconds2) = 0;
   virtual void get_scaling(void* D, void* E, double* c) = 0;
   virtual void comm_init(int nranks, int rank, const void* id128) = 0;
   virtual void p2p_export(void* blob128) = 0;
@@ -214,7 +216,12 @@ class Engine : public EngineBase {
   Engine(const cosmo_b200_problem& p, const cosmo_b200_settings& st);
   ~Engine() override;
   void update_settings(const cosmo_b200_settings& st) override {
-    if (st.sigma != st_.sigma) destroy_cg_graphs();   // sigma is baked into the captured kernel arguments
+    if (st.kkt_solver == COSMO_B200_KKT_DIRECT && !d_L_.p)
+      throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "kkt_solver DIRECT is chosen when the engine is created (its factor is set up there)"};
+    if (st.sigma != st_.sigma) {
+      destroy_cg_graphs();   // sigma is baked into the captured kernel arguments
+      d_stale_ = true;       // and into the diagonal of the reduced matrix
+    }
     st_ = st;
   }
   void warm_start(const void* x, const void* s, const void* mu) override;
@@ -230,6 +237,11 @@ class Engine : public EngineBase {
   void get_rho_vec(void* out) override;
   void get_w(void* out) override;
   void psd_stats(int64_t* out8) override;
+  void kkt_factor_stats(int64_t* factorizations, double* seconds2) override {
+    *factorizations = d_factorizations_;
+    seconds2[0] = d_init_s_;
+    seconds2[1] = d_update_s_;
+  }
   void get_scaling(void* D, void* E, double* c) override;
   void equilibrate();
   void comm_init(int nranks, int rank, const void* id128) override;
@@ -305,6 +317,24 @@ class Engine : public EngineBase {
   void cg_iteration_launches(const int* done);
   void build_cg_graphs(const int* done);
   void destroy_cg_graphs();
+  // direct solve of the reduced system (direct.cuh): dense fp64 tile Cholesky factor of M = P + sigma I + A'RA
+  int d_NT_ = 0, d_nd_ = 0, d_G_ = 0;
+  long long d_ldg_ = 0;
+  size_t d_smem_ = 0;
+  std::vector<int> d_rows_host_;                  // the dense rows of A (assembled through the panel product)
+  DevBuf<double> d_L_, d_Gt_, d_y_, d_x_, d_dinv_;
+  DevBuf<int> d_rows_, d_fail_;
+  DevBuf<unsigned char> d_dense_;
+  DevBuf<unsigned> d_ready_;
+  unsigned d_epoch_ = 0;
+  bool d_stale_ = true;                           // rho or sigma changed since the last factorisation
+  long long d_factorizations_ = 0;
+  double d_init_s_ = 0.0, d_update_s_ = 0.0;      // init_factor_time / factor_update_time (types.jl:31-32)
+  void direct_plan(const HostCsr& a, const HostCsr& p);
+  void direct_alloc();
+  void direct_factor();
+  void direct_solve();
+  void ensure_factor() { if (st_.kkt_solver == COSMO_B200_KKT_DIRECT && d_stale_) direct_factor(); }
   long long kkt_counter_ = 1;   // S.iteration_counter
   int last_cg_iters_ = 1;
   long long total_inner_ = 0, total_mults_ = 0;
@@ -820,6 +850,10 @@ Engine<T>::Engine(const cosmo_b200_problem& p, const cosmo_b200_settings& st) : 
     HostCsr a, at, pp, ppt;
     csc_to_host_csrs<T>(p.A, p.index_base, a, at);
     lap("csc -> csr (A, A')");
+    if (st_.kkt_solver == COSMO_B200_KKT_DIRECT) {   // memory gate before anything of the problem is allocated
+      csc_to_host_csrs<T>(p.P, p.index_base, pp, ppt);
+      direct_plan(a, pp);
+    }
     build_csr(A_, a);
     lap("upload csr A");
     build_windows(A_, a);
@@ -906,6 +940,10 @@ Engine<T>::Engine(const cosmo_b200_problem& p, const cosmo_b200_settings& st) : 
   }
   classify_and_set_rho(true);
   sync();
+  if (st_.kkt_solver == COSMO_B200_KKT_DIRECT) {   // the initial factorisation of setup! (setup.jl:56)
+    direct_alloc();
+    direct_factor();
+  }
   create_time_ = now_s() - t_ctor0;
   auto_rho_interval_ = 0;
 }
@@ -961,6 +999,7 @@ void Engine<T>::classify_and_set_rho(bool reset_rho, bool rebuild_vec) {
   }
   rho_vec_kernel<T><<<vgrid(m_), kBlock, 0, stream_>>>(m_, rho_class_.p, (T)rho_, (T)st_.RHO_EQ_OVER_RHO_INEQ, (T)st_.RHO_MIN, rho_vec_.p);
   check_launch("rho_vec");
+  d_stale_ = true;
 }
 
 // scale_ruiz! (scaling.jl:21-116) on the resident data; see ruiz.cuh
@@ -1074,6 +1113,7 @@ template <typename T>
 void Engine<T>::update_rho(const void* rho_vec, double rho) {
   if (rho_vec) upload_vec(rho_vec_, rho_vec, m_);
   rho_ = rho;
+  d_stale_ = true;
   sync();
 }
 
@@ -1110,6 +1150,8 @@ void Engine<T>::allreduce_max(T* buf, size_t count) {
 template <typename T>
 void Engine<T>::comm_init(int nranks, int rank, const void* id128) {
   if (nranks < 1 || rank < 0 || rank >= nranks) throw EngineError{COSMO_B200_ERR_INVALID, "bad rank / nranks"};
+  if (nranks > 1 && st_.kkt_solver == COSMO_B200_KKT_DIRECT)
+    throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "the direct KKT solver is single-GPU (use CG or MINRES when sharded)"};
   nranks_ = nranks; rank_ = rank;
   if (nranks == 1) return;
   std::string e;
@@ -1275,8 +1317,11 @@ template <typename T>
 void Engine<T>::kkt_core(bool fused_tail, const T* w_src, T* w_dst) {
   const bool lead = (rank_ == 0);
   const bool full = (st_.kkt_solver == COSMO_B200_KKT_MINRES);
-  if (st_.kkt_solver != COSMO_B200_KKT_CG && st_.kkt_solver != COSMO_B200_KKT_MINRES_REDUCED && !full)
+  const bool direct = (st_.kkt_solver == COSMO_B200_KKT_DIRECT);
+  if (st_.kkt_solver != COSMO_B200_KKT_CG && st_.kkt_solver != COSMO_B200_KKT_MINRES_REDUCED && !full && !direct)
     throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "unknown kkt_solver"};
+  if (direct && nranks_ > 1)
+    throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "the direct KKT solver is single-GPU (use CG or MINRES when sharded)"};
   if (full && nranks_ > 1)
     throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "full-KKT MINRES is single-GPU in this build (use CG or reduced MINRES when sharded)"};
   if (full) {
@@ -1292,6 +1337,7 @@ void Engine<T>::kkt_core(bool fused_tail, const T* w_src, T* w_dst) {
               EpiAddVec<T>{nullptr, rhsb_.p, lead ? ls_.p : nullptr}, red(SC_TMP0), "spmv_rhs");
   allreduce_sum(rhsb_.p, n_);
   if (st_.kkt_solver == COSMO_B200_KKT_CG) kkt_cg(isc_.p + ISC_DONE);
+  else if (direct) direct_solve();
   else kkt_minres(false);
   kkt_counter_ += 1;
   if (fused_tail) {
@@ -1494,6 +1540,141 @@ void Engine<T>::kkt_minres(bool full) {
   }
 }
 
+// ---- direct solve of the reduced system (direct.cuh) ------------------------------------------------------------
+// Sizes the factor and its workspace from the host copies of A and P, before anything is allocated: refuses when they
+// need more than half of the free device memory (the GPU may be shared; the caller falls back to an indirect solver).
+template <typename T>
+void Engine<T>::direct_plan(const HostCsr& a, const HostCsr& p) {
+  // one warp adds a row's entries in parallel: duplicate entries inside a row would race
+  for (const HostCsr* h : {&a, &p})
+    for (int r = 0; r < h->nrows; ++r)
+      for (int k = h->rowptr[r] + 1; k < h->rowptr[r + 1]; ++k)
+        if (h->col[k] == h->col[k - 1])
+          throw EngineError{COSMO_B200_ERR_INVALID, "the direct KKT solver needs A and P without duplicate entries"};
+  d_NT_ = std::max(1, (n_ + direct::NB - 1) / direct::NB);
+  d_rows_host_.clear();
+  for (int i = 0; i < a.nrows; ++i)
+    if (direct::dense_row(a.rowptr[i + 1] - a.rowptr[i], n_)) d_rows_host_.push_back(i);
+  d_nd_ = (int)d_rows_host_.size();
+  d_ldg_ = (long long)(d_nd_ + direct::NB - 1) / direct::NB * direct::NB;
+  const double npad = (double)d_NT_ * direct::NB;
+  const double need = 8.0 * (double)direct::tile_off(d_NT_, 0) + 8.0 * npad * (double)d_ldg_ + 16.0 * npad +
+                      8.0 * d_NT_ + (double)m_ + 4.0 * d_nd_;
+  size_t free_b = 0, total_b = 0;
+  CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+  if (need > 0.5 * (double)free_b) {
+    char b[320];
+    snprintf(b, sizeof(b), "the direct KKT solver needs %.0f bytes for its dense factor (n = %d) and workspace, more than half of "
+             "the %zu bytes of free device memory: use an indirect kkt_solver", need, n_, free_b);
+    throw EngineError{COSMO_B200_ERR_UNSUPPORTED, b};
+  }
+}
+
+template <typename T>
+void Engine<T>::direct_alloc() {
+  const int NT = d_NT_;
+  d_L_.alloc(direct::tile_off(NT, 0), false);
+  if (d_nd_) {
+    d_Gt_.alloc((size_t)NT * direct::NB * d_ldg_, false);
+    d_rows_.upload(d_rows_host_, stream_);
+  }
+  std::vector<unsigned char> dense(std::max(m_, 1), 0);
+  for (int i : d_rows_host_) dense[i] = 1;
+  d_dense_.upload(dense, stream_);
+  d_y_.alloc((size_t)NT * direct::NB);
+  d_x_.alloc((size_t)NT * direct::NB);
+  d_dinv_.alloc((size_t)NT * direct::NB);
+  d_ready_.alloc(2 * (size_t)NT);
+  d_fail_.alloc(1);
+  d_epoch_ = 0;
+  CUDA_TRY(cudaFuncSetAttribute(direct::trsm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)direct::kPanelSmem));
+  // persistent sweep grid: at most two CTAs per SM, all co-resident (cooperative launch)
+  int coop = 0;
+  CUDA_TRY(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device_));
+  if (!coop) throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "the direct KKT solver needs cooperative launches"};
+  d_G_ = 0;
+  for (int per_sm = 2; per_sm >= 1 && d_G_ == 0; --per_sm) {
+    const int G = std::min(NT, per_sm * num_sms_);
+    const int R = (NT + G - 1) / G;
+    const size_t smem = direct::trsv_smem_bytes(R);
+    CUDA_TRY(cudaFuncSetAttribute(direct::trsv_persistent_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int nb = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, direct::trsv_persistent_kernel<T>, direct::kThreads, smem));
+    if (nb >= per_sm || (G <= num_sms_ && nb >= 1)) { d_G_ = G; d_smem_ = smem; }
+  }
+  if (d_G_ == 0) throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "the direct KKT solver's sweep kernel does not fit on an SM"};
+  sync();
+}
+
+// assemble M = P + sigma I + A' R A and factor it (right-looking tile Cholesky); one host synchronisation for the
+// pivot check, at the reference's own decision points (setup!, update_rho!)
+template <typename T>
+void Engine<T>::direct_factor() {
+  const int NT = d_NT_, Npad = NT * direct::NB;
+  cudaEvent_t ev[3];
+  for (auto& e : ev) CUDA_TRY(cudaEventCreate(&e));
+  CUDA_TRY(cudaEventRecord(ev[0], stream_));
+  CUDA_TRY(cudaMemsetAsync(d_L_.p, 0, direct::tile_off(NT, 0) * sizeof(double), stream_));
+  CUDA_TRY(cudaMemsetAsync(d_fail_.p, 0, sizeof(int), stream_));
+  direct::assemble_sparse_kernel<T><<<(int)(((long long)Npad * 32 + direct::kThreads - 1) / direct::kThreads), direct::kThreads, 0,
+                                      stream_>>>(n_, Npad, d_L_.p, P_.view(), At_.view(), A_.view(), rho_vec_.p, d_dense_.p, st_.sigma);
+  check_launch("direct_assemble_sparse");
+  if (d_nd_) {
+    CUDA_TRY(cudaMemsetAsync(d_Gt_.p, 0, (size_t)Npad * d_ldg_ * sizeof(double), stream_));
+    direct::gather_dense_kernel<T><<<d_nd_, direct::kThreads, 0, stream_>>>(d_rows_.p, d_ldg_, A_.view(), rho_vec_.p, d_Gt_.p);
+    check_launch("direct_gather_dense");
+    direct::tile_update_kernel<true><<<(unsigned)((long long)NT * (NT + 1) / 2), direct::kThreads, 0, stream_>>>(
+        d_L_.p, NT, 0, 0, d_Gt_.p, d_ldg_, 1.0);
+    check_launch("direct_assemble_dense");
+  }
+  CUDA_TRY(cudaEventRecord(ev[1], stream_));
+  for (int K = 0; K < NT; ++K) {
+    direct::potrf_kernel<<<1, direct::kThreads, direct::kPanelSmem / 2, stream_>>>(d_L_.p, d_dinv_.p, K, d_fail_.p);
+    check_launch("direct_potrf");
+    const long long c = NT - K - 1;
+    if (c > 0) {
+      direct::trsm_kernel<<<(unsigned)c, direct::kThreads, direct::kPanelSmem, stream_>>>(d_L_.p, K);
+      check_launch("direct_trsm");
+      direct::tile_update_kernel<false><<<(unsigned)(c * (c + 1) / 2), direct::kThreads, 0, stream_>>>(d_L_.p, NT, K + 1, K, nullptr, 0, -1.0);
+      check_launch("direct_update");
+    }
+  }
+  CUDA_TRY(cudaEventRecord(ev[2], stream_));
+  int fail = 0;
+  CUDA_TRY(cudaMemcpyAsync(&fail, d_fail_.p, sizeof(int), cudaMemcpyDeviceToHost, stream_));
+  sync();
+  float ms_asm = 0.f, ms_fac = 0.f;
+  CUDA_TRY(cudaEventElapsedTime(&ms_asm, ev[0], ev[1]));
+  CUDA_TRY(cudaEventElapsedTime(&ms_fac, ev[1], ev[2]));
+  for (auto& e : ev) cudaEventDestroy(e);
+  if (getenv("COSMO_B200_SETUP_DEBUG"))
+    fprintf(stderr, "[direct] n %d NT %d dense rows %d assembly %.3f ms factorisation %.3f ms pivot failure in tile column %d\n",
+            n_, NT, d_nd_, ms_asm, ms_fac, fail - 1);
+  // positive_inertia(ldlfact) == n || error(...) (kktsolver.jl:304): inertia (n, m, 0) <=> M positive definite
+  if (fail) throw EngineError{COSMO_B200_ERR_INVALID, "Objective function is not convex."};
+  const double sec = 1e-3 * ((double)ms_asm + (double)ms_fac);
+  if (d_factorizations_ == 0) d_init_s_ = sec; else d_update_s_ += sec;
+  ++d_factorizations_;
+  d_stale_ = false;
+}
+
+// xsol_ = M^-1 rhsb_ : both triangular sweeps in one cooperative launch
+template <typename T>
+void Engine<T>::direct_solve() {
+  if (++d_epoch_ == 0) {   // the ready flags carry the epoch: clear them once per 2^32 solves
+    CUDA_TRY(cudaMemsetAsync(d_ready_.p, 0, 2 * (size_t)d_NT_ * sizeof(unsigned), stream_));
+    d_epoch_ = 1;
+  }
+  direct::TrsvArgs<T> a;
+  a.L = d_L_.p; a.dinv = d_dinv_.p; a.n = n_; a.NT = d_NT_; a.G = d_G_;
+  a.rhs = rhsb_.p; a.out = xsol_.p; a.y = d_y_.p; a.x = d_x_.p;
+  a.ready_f = d_ready_.p; a.ready_b = d_ready_.p + d_NT_; a.epoch = d_epoch_;
+  void* args[] = {&a};
+  CUDA_TRY(cudaLaunchCooperativeKernel((const void*)direct::trsv_persistent_kernel<T>, dim3(d_G_), dim3(direct::kThreads), args,
+                                       d_smem_, stream_));
+  check_launch("direct_trsv");
+}
+
 // calculate_residuals! + max_res_component_norm + calculate_cost! (residuals.jl:30-96, 143-147)
 template <typename T>
 void Engine<T>::compute_residuals(const T* x, const T* s, const T* mu, bool ignore_scaling, double out[5]) {
@@ -1535,6 +1716,7 @@ bool Engine<T>::adapt_rho(const T* x) {
     rho_ = new_rho;
     rho_vec_kernel<T><<<vgrid(m_), kBlock, 0, stream_>>>(m_, rho_class_.p, (T)rho_, (T)st_.RHO_EQ_OVER_RHO_INEQ, (T)st_.RHO_MIN, rho_vec_.p);
     check_launch("rho_vec");
+    d_stale_ = true;   // update_rho! refactors (parameters.jl:86), lazily before the next solve
     rho_updates_.push_back(new_rho);
     return true;
   }
@@ -1776,6 +1958,7 @@ void Engine<T>::solve(cosmo_b200_result* out) {
     }
     // the tail reads w_s from ws_rhs's buffer and writes W[dst] (elementwise, may alias)
     T* wd = W_[dst].p;
+    ensure_factor();
     t_kkt_.begin(stream_);
     kkt_core(true, ws_override ? (ws_override - n) : w, wd);
     t_kkt_.end(stream_);
@@ -1971,6 +2154,7 @@ void Engine<T>::kkt_solve(const void* rhs, void* sol, int64_t* inner) {
   upload_vec(ls_, rhs, (size_t)n_ + m_);
   scale_kernel<T><<<vgrid(m_), kBlock, 0, stream_>>>(m_, rho_vec_.p, ls_.p + n_, t0_.p);
   check_launch("scale_x2");
+  ensure_factor();
   kkt_core(false, nullptr, nullptr);
   download_vec(sol, xsol_.p, n_);
   download_vec(static_cast<T*>(sol) + n_, nu_.p, m_);
@@ -1978,7 +2162,7 @@ void Engine<T>::kkt_solve(const void* rhs, void* sol, int64_t* inner) {
   if (inner) {
     CUDA_TRY(cudaMemcpyAsync(h_isc_, isc_.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, stream_));
     sync();
-    *inner = h_isc_[ISC_IT];
+    *inner = st_.kkt_solver == COSMO_B200_KKT_DIRECT ? 0 : h_isc_[ISC_IT];
   }
 }
 
@@ -2162,6 +2346,10 @@ int cosmo_b200_psd_stats(cosmo_b200_handle* h, int64_t out[8]) {
 }
 int cosmo_b200_get_scaling(cosmo_b200_handle* h, void* D, void* E, double* c) {
   ABI_GUARD(h, h->impl->get_scaling(D, E, c));
+}
+int cosmo_b200_kkt_factor_stats(cosmo_b200_handle* h, int64_t* factorizations, double seconds[2]) {
+  if (!factorizations || !seconds) return COSMO_B200_ERR_INVALID;
+  ABI_GUARD(h, h->impl->kkt_factor_stats(factorizations, seconds));
 }
 int cosmo_b200_comm_unique_id(void* id128) {
   if (!id128) return COSMO_B200_ERR_INVALID;

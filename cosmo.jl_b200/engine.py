@@ -21,7 +21,7 @@ F64, F32 = 0, 1
 ZERO, NONNEG, BOX, SOC, PSD_SQUARE, PSD_TRIANGLE, EXP, DUAL_EXP, POW, DUAL_POW, PSD_TRIANGLE_COMPLEX = range(11)
 STATUS = {0: "Undetermined", 1: "Solved", 2: "Max_iter_reached", 3: "Time_limit_reached",
           4: "Primal_infeasible", 5: "Dual_infeasible", 6: "Unsolved"}
-KKT_CG, KKT_MINRES_REDUCED, KKT_MINRES = 0, 1, 2
+KKT_CG, KKT_MINRES_REDUCED, KKT_MINRES, KKT_DIRECT = 0, 1, 2, 3
 ACC_EMPTY, ACC_ANDERSON = 0, 1
 
 
@@ -86,7 +86,7 @@ EXPORTS = [
     "cosmo_b200_update_rho", "cosmo_b200_reset", "cosmo_b200_solve", "cosmo_b200_project", "cosmo_b200_kkt_solve",
     "cosmo_b200_residuals", "cosmo_b200_spmv", "cosmo_b200_spmv_bench", "cosmo_b200_get_rho_vec", "cosmo_b200_get_w",
     "cosmo_b200_comm_unique_id", "cosmo_b200_comm_init", "cosmo_b200_comm_p2p_export", "cosmo_b200_comm_p2p_attach",
-    "cosmo_b200_tc_gemm_test", "cosmo_b200_psd_stats", "cosmo_b200_get_scaling",
+    "cosmo_b200_tc_gemm_test", "cosmo_b200_psd_stats", "cosmo_b200_get_scaling", "cosmo_b200_kkt_factor_stats",
 ]
 
 _lib = None
@@ -134,6 +134,7 @@ def load_library(rebuild_if_stale=True):
     lib.cosmo_b200_comm_p2p_attach.argtypes = [vp, vp, C.c_int32]
     lib.cosmo_b200_psd_stats.argtypes = [vp, C.POINTER(C.c_int64)]
     lib.cosmo_b200_get_scaling.argtypes = [vp, vp, vp, C.POINTER(C.c_double)]
+    lib.cosmo_b200_kkt_factor_stats.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_double)]
     lib.cosmo_b200_tc_gemm_test.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp, vp, C.c_int32,
                                             C.POINTER(C.c_double), C.POINTER(C.c_double)]
     for name in EXPORTS:
@@ -389,6 +390,14 @@ class Engine:
         keys = ("tc_projections", "tc_fallbacks", "tc_last_steps", "tc_last_checks", "sign_projections", "sign_fallbacks",
                 "jacobi_last_sweeps", "tc_slices")
         return dict(zip(keys, [int(v) for v in out]))
+
+    def kkt_factor_stats(self):
+        """Factorisations of the direct KKT solver (cosmo_b200_kkt_factor_stats): their count, the device seconds of the
+        initial one (init_factor_time) and of all later ones (factor_update_time); zeros on an indirect solver."""
+        cnt = C.c_int64(0)
+        sec = (C.c_double * 2)()
+        self._check(self._lib.cosmo_b200_kkt_factor_stats(self._h, C.byref(cnt), sec))
+        return {"factorizations": int(cnt.value), "init_factor_time": float(sec[0]), "factor_update_time": float(sec[1])}
 
 
 def tc_gemm(A, B, slices=8, groups=0, reps=0):

@@ -224,7 +224,7 @@ class Settings:
     max_iter: int = 5000
     verbose: bool = False
     verbose_timing: bool = False             # settings.jl:43: here it forces the device phase timers (proj_time, kkt_time)
-    kkt_solver: str = "CGIndirectKKTSolver"   # the engine implements the indirect family only
+    kkt_solver: str = "CGIndirectKKTSolver"   # the indirect family, or "DirectReducedKKTSolver" (dense device Cholesky)
     check_termination: int = 25
     check_infeasibility: int = 40
     scaling: int = 10
@@ -262,13 +262,14 @@ class Settings:
     compact_transformation: bool = True         # the only transformation restated
 
     _KKT = {"CGIndirectKKTSolver": _eng.KKT_CG, "MINRESIndirectKKTSolver": _eng.KKT_MINRES,
-            "IndirectReducedKKTSolver:MINRES": _eng.KKT_MINRES_REDUCED}
+            "IndirectReducedKKTSolver:MINRES": _eng.KKT_MINRES_REDUCED, "DirectReducedKKTSolver": _eng.KKT_DIRECT}
 
     def to_struct(self) -> "_eng.SettingsStruct":
         if self.kkt_solver not in self._KKT:
             raise _eng.EngineError(_eng.ERR_UNSUPPORTED,
                                    "kkt_solver %r is a direct CPU factorisation; the B200 engine implements "
-                                   "CGIndirectKKTSolver / MINRESIndirectKKTSolver" % self.kkt_solver)
+                                   "CGIndirectKKTSolver / MINRESIndirectKKTSolver, and DirectReducedKKTSolver for an "
+                                   "exact solve on the device" % self.kkt_solver)
         if self.accelerator not in ("EmptyAccelerator", "AndersonAccelerator"):
             raise _eng.EngineError(_eng.ERR_UNSUPPORTED,
                                    "accelerator %r: the engine implements EmptyAccelerator and AndersonAccelerator"
@@ -587,6 +588,9 @@ class Model:
             x, s, mu = _chordal.reverse(self._dec, x, s, mu, complete_dual=self.settings.complete_dual)
         self.x, self.s, self.mu = x.copy(), s.copy(), mu.copy()
         times = dict(out.times)
+        if self.settings.kkt_solver == "DirectReducedKKTSolver":
+            fs = self.engine.kkt_factor_stats()
+            times["init_factor_time"], times["factor_update_time"] = fs["init_factor_time"], fs["factor_update_time"]
         times["setup_time"] = setup_time
         times["solver_time"] = time.perf_counter() - t0
         info = ResultInfo(out.r_prim, out.r_dual, out.max_norm_prim, out.max_norm_dual, list(out.rho_updates))

@@ -89,11 +89,18 @@ enum {
 /* accelerators (COSMOAccelerators.jl types selectable through settings.accelerator) */
 enum { COSMO_B200_ACC_EMPTY = 0, COSMO_B200_ACC_ANDERSON = 1 };
 
-/* KKT plugins (src/linear_solver/kktsolver_indirect.jl:173-189) */
+/* KKT plugins (src/linear_solver/kktsolver_indirect.jl:173-189; kktsolver.jl:285-349) */
 enum {
   COSMO_B200_KKT_CG = 0,             /* CGIndirectKKTSolver      (reduced system, CG)      :3-88   */
   COSMO_B200_KKT_MINRES_REDUCED = 1, /* IndirectReducedKKTSolver(solver_type = :MINRES)    :3-88   */
-  COSMO_B200_KKT_MINRES = 2          /* MINRESIndirectKKTSolver  (full KKT, MINRES)        :90-162 */
+  COSMO_B200_KKT_MINRES = 2,         /* MINRESIndirectKKTSolver  (full KKT, MINRES)        :90-162 */
+  COSMO_B200_KKT_DIRECT = 3          /* the engine's counterpart of QdldlKKTSolver / CholmodKKTSolver (kktsolver.jl:285-349):
+                                        exact solves through a dense fp64 Cholesky factor of the reduced matrix
+                                        P + sigma I + A' diag(rho) A, factored at create and again after every change of
+                                        rho or sigma.  Chosen at create; single-GPU; refused (ERR_UNSUPPORTED) when the
+                                        factor would need more than half of the free device memory, and with
+                                        "Objective function is not convex." (ERR_INVALID) when the matrix is not
+                                        positive definite. */
 };
 
 /* SparseMatrixCSC{T,Int64} as Julia stores it */
@@ -238,7 +245,8 @@ int cosmo_b200_solve(cosmo_b200_handle* h, cosmo_b200_result* out);
 /* ---- plugin-granularity entry points (also the parity-test hooks) -------- */
 /* project!(s, C): s_out = Pi_K(w_s) (convexset.jl:885-891) */
 int cosmo_b200_project(cosmo_b200_handle* h, const void* w_s, void* s_out);
-/* solve!(kkt_solver, sol, rhs): rhs, sol in R^{n+m} (kktsolver_indirect.jl:36-88,123-162) */
+/* solve!(kkt_solver, sol, rhs): rhs, sol in R^{n+m} (kktsolver_indirect.jl:36-88,123-162; kktsolver.jl:315-320);
+   inner_iterations = 0 for the direct solver */
 int cosmo_b200_kkt_solve(cosmo_b200_handle* h, const void* rhs, void* sol, int64_t* inner_iterations);
 /* calculate_residuals! + max_res_component_norm + calculate_cost! (residuals.jl:30-96,143-147)
    for given (x, s, mu); out = {r_prim, r_dual, max_norm_prim, max_norm_dual, cost} */
@@ -273,6 +281,11 @@ int cosmo_b200_comm_p2p_attach(cosmo_b200_handle* h, const void* blobs, int32_t 
    block Jacobi, Newton-Schulz steps of the last one, weighted-residual checks of the last one, FP64-FMA sign
    projections, their fallbacks, block-Jacobi sweeps of the last eigensolve, int8 slices per operand}. */
 int cosmo_b200_psd_stats(cosmo_b200_handle* h, int64_t out[8]);
+/* The direct KKT solver's factorisations (ws.times.init_factor_time / factor_update_time, types.jl:31-32):
+   factorizations = number of factorisations so far; seconds[0] = device time of the initial one (at create),
+   seconds[1] = device time of all later ones (after rho / sigma changes), assembly of the reduced matrix included.
+   A handle on an indirect solver reports 0 and zeros. */
+int cosmo_b200_kkt_factor_stats(cosmo_b200_handle* h, int64_t* factorizations, double seconds[2]);
 /* The product kernel of the large-cone PSD projection on its own: C = A B for symmetric, commuting N x N fp64
    matrices (column-major) through `k` int8 slices on tcgen05 (csrc/tc_gemm.cuh; the reference's counterpart is the
    BLAS-3 part of project!(::PsdCone), convexset.jl:244-260).  `groups` = number of slice-pair groups kept
