@@ -32,6 +32,7 @@
 #include "ruiz.cuh"
 #include "cg_persistent.cuh"
 #include "direct.cuh"
+#include "ldl_symbolic.h"
 
 namespace cosmo {
 
@@ -2431,6 +2432,51 @@ int cosmo_b200_tc_gemm_test(int32_t N, int32_t k, int32_t kstep, int32_t gpb, co
   cudaFree(A_d); cudaFree(B_d); cudaFree(C_d); cudaFree(coef_d); cudaFree(part_d);
   cudaStreamDestroy(st);
   return rc;
+}
+
+// ---- symbolic analysis of the full KKT matrix (ldl_symbolic.h); host only ---------------------------------------------
+static void kkt_pattern(const cosmo_b200_csc& M, int64_t nrows, int64_t ncols, int base, const char* name,
+                        std::vector<int64_t>& colptr, std::vector<int64_t>& row) {
+  const std::string nm(name);
+  if (M.nrows != nrows || M.ncols != ncols) throw cosmo::EngineError{COSMO_B200_ERR_INVALID, nm + " has the wrong shape"};
+  colptr.assign(ncols + 1, 0);
+  if (ncols > 0 && !M.colptr) throw cosmo::EngineError{COSMO_B200_ERR_INVALID, nm + ": null colptr"};
+  for (int64_t j = 0; j <= ncols; ++j) {
+    const int64_t v = ncols ? M.colptr[j] - base : 0;
+    if (v < 0 || (j > 0 && v < colptr[j - 1])) throw cosmo::EngineError{COSMO_B200_ERR_INVALID, nm + ": colptr not monotone"};
+    colptr[j] = v;
+  }
+  const int64_t nnz = colptr[ncols];
+  if (nnz > 0 && !M.rowval) throw cosmo::EngineError{COSMO_B200_ERR_INVALID, nm + ": null rowval"};
+  row.resize(nnz);
+  std::vector<int64_t> seen(nrows, -1);
+  for (int64_t j = 0; j < ncols; ++j)
+    for (int64_t k = colptr[j]; k < colptr[j + 1]; ++k) {
+      const int64_t i = M.rowval[k] - base;
+      if (i < 0 || i >= nrows) throw cosmo::EngineError{COSMO_B200_ERR_INVALID, nm + ": row index out of range"};
+      if (seen[i] == j) throw cosmo::EngineError{COSMO_B200_ERR_INVALID, nm + " has duplicate entries"};
+      seen[i] = j;
+      row[k] = i;
+    }
+}
+
+int cosmo_b200_kkt_symbolic(const cosmo_b200_problem* prob, int64_t* perm, int64_t info[8]) {
+  if (!prob || !info) { cosmo::g_create_error = "null argument"; return COSMO_B200_ERR_INVALID; }
+  try {
+    if (prob->n < 0 || prob->m < 0 || (prob->index_base != 0 && prob->index_base != 1))
+      throw cosmo::EngineError{COSMO_B200_ERR_INVALID, "bad dimensions or index base"};
+    std::vector<int64_t> pc, pr, ac, ar;
+    kkt_pattern(prob->P, prob->n, prob->n, prob->index_base, "P", pc, pr);
+    kkt_pattern(prob->A, prob->m, prob->n, prob->index_base, "A", ac, ar);
+    const cosmo::ldl::Symbolic S = cosmo::ldl::analyse(prob->n, prob->m, pc, pr, ac, ar);
+    if (perm) std::copy(S.perm.begin(), S.perm.end(), perm);
+    const int64_t out[8] = {S.nnz_L, (int64_t)S.sn_first.size() - 1, S.height, S.widest, S.largest_front,
+                            S.factor_bytes, S.workspace_bytes, S.dense};
+    std::copy(out, out + 8, info);
+    return COSMO_B200_OK;
+  } catch (const cosmo::EngineError& e) { cosmo::g_create_error = e.msg; return e.code; }
+  catch (const std::bad_alloc&) { cosmo::g_create_error = "host allocation failed"; return COSMO_B200_ERR_ALLOC; }
+  catch (...) { cosmo::g_create_error = "unknown error"; return COSMO_B200_ERR_INVALID; }
 }
 
 }  // extern "C"

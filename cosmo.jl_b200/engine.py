@@ -87,6 +87,7 @@ EXPORTS = [
     "cosmo_b200_residuals", "cosmo_b200_spmv", "cosmo_b200_spmv_bench", "cosmo_b200_get_rho_vec", "cosmo_b200_get_w",
     "cosmo_b200_comm_unique_id", "cosmo_b200_comm_init", "cosmo_b200_comm_p2p_export", "cosmo_b200_comm_p2p_attach",
     "cosmo_b200_tc_gemm_test", "cosmo_b200_psd_stats", "cosmo_b200_get_scaling", "cosmo_b200_kkt_factor_stats",
+    "cosmo_b200_kkt_symbolic",
 ]
 
 _lib = None
@@ -135,6 +136,7 @@ def load_library(rebuild_if_stale=True):
     lib.cosmo_b200_psd_stats.argtypes = [vp, C.POINTER(C.c_int64)]
     lib.cosmo_b200_get_scaling.argtypes = [vp, vp, vp, C.POINTER(C.c_double)]
     lib.cosmo_b200_kkt_factor_stats.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_double)]
+    lib.cosmo_b200_kkt_symbolic.argtypes = [C.POINTER(ProblemStruct), vp, C.POINTER(C.c_int64)]
     lib.cosmo_b200_tc_gemm_test.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp, vp, C.c_int32,
                                             C.POINTER(C.c_double), C.POINTER(C.c_double)]
     for name in EXPORTS:
@@ -398,6 +400,38 @@ class Engine:
         sec = (C.c_double * 2)()
         self._check(self._lib.cosmo_b200_kkt_factor_stats(self._h, C.byref(cnt), sec))
         return {"factorizations": int(cnt.value), "init_factor_time": float(sec[0]), "factor_update_time": float(sec[1])}
+
+
+SYMBOLIC_INFO = ("nnz_L", "supernodes", "height", "widest", "largest_front", "factor_bytes", "workspace_bytes", "dense")
+
+
+def kkt_symbolic(P, A):
+    """Symbolic analysis of the full KKT matrix [P + sigma I, A'; A, -R^-1] (cosmo_b200_kkt_symbolic, host only).
+
+    Returns (perm, info): the 0-based elimination order of the n + m nodes (x first, then the rows of A) and a dict
+    with the keys of SYMBOLIC_INFO."""
+    import scipy.sparse as sp
+    lib = load_library()
+    P = sp.csc_matrix(P)
+    A = sp.csc_matrix(A)
+    m, n = A.shape
+    keep = []
+
+    def csc(M):
+        colptr = np.ascontiguousarray(M.indptr, dtype=np.int64)
+        rowval = np.ascontiguousarray(M.indices, dtype=np.int64)
+        keep.extend([colptr, rowval])
+        return CscStruct(M.shape[0], M.shape[1], _ptr(colptr), _ptr(rowval), None)
+
+    prob = ProblemStruct()
+    prob.dtype, prob.index_base, prob.m, prob.n = F64, 0, m, n
+    prob.P, prob.A = csc(P), csc(A)
+    perm = np.empty(n + m, dtype=np.int64)
+    info = (C.c_int64 * 8)()
+    rc = lib.cosmo_b200_kkt_symbolic(C.byref(prob), _ptr(perm), info)
+    if rc != OK:
+        raise EngineError(rc, (lib.cosmo_b200_last_error(None) or b"").decode())
+    return perm, dict(zip(SYMBOLIC_INFO, [int(v) for v in info]))
 
 
 def tc_gemm(A, B, slices=8, groups=0, reps=0):

@@ -286,6 +286,17 @@ int cosmo_b200_psd_stats(cosmo_b200_handle* h, int64_t out[8]);
    seconds[1] = device time of all later ones (after rho / sigma changes), assembly of the reduced matrix included.
    A handle on an indirect solver reports 0 and zeros. */
 int cosmo_b200_kkt_factor_stats(cosmo_b200_handle* h, int64_t* factorizations, double seconds[2]);
+/* Symbolic analysis of the full quasi-definite KKT matrix K = [P + sigma I, A'; A, -R^-1] (the pattern QdldlKKTSolver
+   factors, kktsolver.jl:285-320): approximate minimum degree ordering with dense nodes ordered last, elimination tree,
+   column counts, relaxed supernodes.  Host only: needs no GPU and no handle, reads only the problem's dimensions,
+   index_base and the patterns of P and A (no duplicate entries).  perm (n + m entries, or NULL) receives the
+   elimination order, 0-based: perm[k] is the k-th node eliminated (node j < n is x_j, node n + i is row i of A).
+   info = {nnz(L) including the diagonal, supernodes, height of the supernodal tree, widest supernode (columns),
+   largest front (columns + rows below), factor bytes (fp64 (columns + rows below) x columns per supernode),
+   workspace bytes (fan-in panel, solve vectors, scatter map), nodes postponed as dense}.  The byte counts are those of
+   a supernodal factorisation on the device (DESIGN §3d), which the engine does not have yet.
+   Errors through cosmo_b200_last_error(NULL). */
+int cosmo_b200_kkt_symbolic(const cosmo_b200_problem* prob, int64_t* perm, int64_t info[8]);
 /* The product kernel of the large-cone PSD projection on its own: C = A B for symmetric, commuting N x N fp64
    matrices (column-major) through `k` int8 slices on tcgen05 (csrc/tc_gemm.cuh; the reference's counterpart is the
    BLAS-3 part of project!(::PsdCone), convexset.jl:244-260).  `groups` = number of slice-pair groups kept
