@@ -320,6 +320,7 @@ class Engine : public EngineBase {
   void destroy_cg_graphs();
   // direct solve of the reduced system (direct.cuh): dense fp64 tile Cholesky factor of M = P + sigma I + A'RA
   int d_NT_ = 0, d_nd_ = 0, d_G_ = 0;
+  int d_ctas_cap_ = 0;                            // COSMO_B200_DIRECT_CTAS: upper bound of the sweep grid (0: none)
   long long d_ldg_ = 0;
   size_t d_smem_ = 0;
   std::vector<int> d_rows_host_;                  // the dense rows of A (assembled through the panel product)
@@ -740,6 +741,8 @@ Engine<T>::Engine(const cosmo_b200_problem& p, const cosmo_b200_settings& st) : 
     use_persistent_ = !(np_ && np_[0] == '1');
     const char* pc = getenv("COSMO_B200_PERSIST_CTAS");
     if (pc && atoi(pc) > 0) persist_ctas_per_sm_ = atoi(pc);
+    const char* dc = getenv("COSMO_B200_DIRECT_CTAS");
+    if (dc && atoi(dc) > 0) d_ctas_cap_ = atoi(dc);
     const char* gm = getenv("COSMO_B200_GRAPH_MULTI");
     graph_multi_ = !(gm && gm[0] == '0');
     const char* g = getenv("COSMO_B200_WIN_GROUP");
@@ -1589,13 +1592,14 @@ void Engine<T>::direct_alloc() {
   d_fail_.alloc(1);
   d_epoch_ = 0;
   CUDA_TRY(cudaFuncSetAttribute(direct::trsm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)direct::kPanelSmem));
-  // persistent sweep grid: at most two CTAs per SM, all co-resident (cooperative launch)
+  // persistent sweep grid: at most two CTAs per SM and at most COSMO_B200_DIRECT_CTAS, all co-resident (cooperative launch)
   int coop = 0;
   CUDA_TRY(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device_));
   if (!coop) throw EngineError{COSMO_B200_ERR_UNSUPPORTED, "the direct KKT solver needs cooperative launches"};
   d_G_ = 0;
   for (int per_sm = 2; per_sm >= 1 && d_G_ == 0; --per_sm) {
-    const int G = std::min(NT, per_sm * num_sms_);
+    int G = std::min(NT, per_sm * num_sms_);
+    if (d_ctas_cap_ > 0) G = std::min(G, d_ctas_cap_);
     const int R = (NT + G - 1) / G;
     const size_t smem = direct::trsv_smem_bytes(R);
     CUDA_TRY(cudaFuncSetAttribute(direct::trsv_persistent_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

@@ -170,6 +170,72 @@ def test_not_positive_definite_is_detected():
         factor(F)
 
 
+def _sweep_schedule(NT, G):
+    """The tile-row ownership arithmetic of trsv_persistent_kernel, in C integer division (every operand is >= 0):
+    for each CTA g, the (step, row) updates of the forward and the backward sweep in program order, with the acc slot each
+    one writes, and the slot each step's owner solves."""
+    fwd, bwd, owner_slots = [], [], []
+    for g in range(G):
+        nrows = (NT - g + G - 1) // G                           # tile rows I = g + G r, r < nrows
+        for J in range(NT):
+            r0 = (J + 1 - g + G - 1) // G if J + 1 > g else 0   # first owned row > J
+            if J % G == g:
+                owner_slots.append((J, g, J // G))
+            for r in range(r0, nrows):
+                fwd.append((g, J, g + G * r, r))                # acc_I -= L(I, J) y_J
+        for I in range(NT - 1, -1, -1):
+            rl = (I - 1 - g) // G if I - 1 >= g else -1         # last owned row < I
+            if I % G == g:
+                owner_slots.append((I, g, I // G))
+            for r in range(rl, -1, -1):
+                bwd.append((g, I, g + G * r, r))                # acc_J -= L(I, J)' x_I
+    return fwd, bwd, owner_slots
+
+
+def test_sweep_ownership_visits_every_tile_once_in_the_order_of_one_row_per_cta():
+    """Every sum of the sweeps runs in an order that does not depend on the grid size G: for each tile row the forward
+    sweep subtracts L(I, J) y_J for J ascending and the backward sweep L(I, J)' x_I for I descending, whichever CTA owns
+    the row and whatever else it owns.  This is why a solve is bitwise the same for every G
+    (tests/test_gpu_direct_kkt_edges.py checks that on the device)."""
+    for NT in range(1, 61):
+        pairs = {(I, J) for I in range(NT) for J in range(I)}
+        for G in range(1, NT + 1):
+            R = -(-NT // G)                                          # acc slots per CTA (trsv_smem_bytes)
+            fwd, bwd, owner_slots = _sweep_schedule(NT, G)
+            # each owned row is the CTA's own row of its slot, and the slot fits in acc
+            for g, J, I, r in fwd + bwd:
+                assert I % G == g and g + G * r == I and 0 <= r < R
+            for step, g, slot in owner_slots:
+                assert g + G * slot == step and slot < R
+            assert sorted(s for s, _, _ in owner_slots) == sorted(list(range(NT)) * 2)   # one owner per step and sweep
+            # forward: pairs (row I, column J), J < I; backward: pairs (row J, column I), J < I -- each exactly once
+            f = [(I, J) for _, J, I, _ in fwd]
+            b = [(I, J) for _, I, J, _ in bwd]
+            assert len(f) == len(set(f)) and set(f) == pairs, (NT, G)
+            assert len(b) == len(set(b)) and set(b) == pairs, (NT, G)
+            # per row: the forward updates in ascending J, the backward ones in descending I
+            f_row, b_row = {r: [] for r in range(NT)}, {r: [] for r in range(NT)}
+            for I, J in f:
+                f_row[I].append(J)
+            for I, J in b:
+                b_row[J].append(I)
+            for row in range(NT):
+                assert f_row[row] == list(range(row)) and b_row[row] == list(range(NT - 1, row, -1)), (NT, G, row)
+            # the forward prefetch (tile (I0, J), I0 = g + G r0) is the first row of step J the update loop visits, and the
+            # backward one (tile (I, J0), J0 = g + G rl) the first of step I
+            first_f, first_b = {}, {}
+            for g, J, I, _ in fwd:
+                first_f.setdefault((g, J), I)
+            for g, I, J, _ in bwd:
+                first_b.setdefault((g, I), J)
+            for g in range(G):
+                for step in range(NT):
+                    r0 = (step + 1 - g + G - 1) // G if step + 1 > g else 0
+                    rl = (step - 1 - g) // G if step - 1 >= g else -1
+                    assert first_f.get((g, step), g + G * r0) == g + G * r0
+                    assert first_b.get((g, step), g + G * rl) == g + G * rl
+
+
 def test_dense_row_rule():
     # the portfolio problem's 2000 rows of F' (10 000 entries) and all-ones row go through the panel product at
     # n = 20 000; its identity and diagonal rows, and rows of a few hundred entries at n = 50 000, stay sparse
